@@ -259,14 +259,16 @@ def run_reference(args, rank):
         for p, (m, s) in zip(params, state):
             adabelief_step(p.data, p.grad, m, s, i, 1e-3, 0.95, 0.99, 1e-6)
             p.grad = None
-        return loss.item()
+        return loss
 
     for i in range(args.warmup):
         step(i + 1)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        step(args.warmup + i + 1)
+        loss = step(args.warmup + i + 1)
     dt = (time.perf_counter() - t0) / max(args.steps, 1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, loss, model)
     value = sample / dt
     print(json.dumps({
         "metric": METRIC, "value": value, "unit": "images/s", "impl": "reference", "n_gpus": args.gpus, "steps": args.steps,
@@ -436,6 +438,30 @@ def roofline_leg(K, run_step, opt_step, n_params: int, step_ms: float, images: i
     return roof
 
 
+DUMP_BUDGET_BYTES = 60_000_000     # under 64 MB (10^6 bytes) in all, .npy headers included
+
+
+def dump_outputs(out_dir: str, loss, model) -> None:
+    """Writes what the last timed step computed, as float32 .npy files in `out_dir`: ``loss`` and ``state.<key>`` for every
+    floating-point entry of the model's state_dict (parameters after the update, normalisation statistics). When the state
+    exceeds the budget, every tensor is cut to the same fraction by a fixed, seeded sample of its flattened elements, so
+    that two runs with the same arguments write the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    state = {f"state.{k}": v.detach() for k, v in model.state_dict().items() if v.is_floating_point()}
+    frac = min(1.0, DUMP_BUDGET_BYTES / (4 * sum(v.numel() for v in state.values())))
+    g = torch.Generator().manual_seed(0)
+    arrays = {"loss": loss.detach().float().reshape(())}
+    for k, v in state.items():
+        if frac < 1.0:
+            idx = torch.randperm(v.numel(), generator=g)[:max(1, int(v.numel() * frac))].sort().values
+            v = v.reshape(-1)[idx.to(v.device)]
+        arrays[k] = v.float()
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v.cpu().numpy())
+    print(f"[bench] wrote {len(arrays)} arrays to {out_dir} (state sampled at {frac:.3f})", file=sys.stderr)
+
+
 TRAIN_MACS = {"repvgg_a0": 2.821e9, "repvgg_a1": 4.329e9, "rexnet1_0x": 0.398e9, "yolov4": 45.52e9, "unet3p": 195.49e9,
               "resnet50": 4.09e9, "resnet18": 1.81e9, "mobileone_s0": 1.07e9}
 
@@ -551,6 +577,8 @@ def measure(args, wl: Workload, rank: int, local_rank: int, world: int, full: bo
     e3.record()
     barrier()
     ms_e2e = e2.elapsed_time(e3) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model)
 
     if world > 1:
         tt = torch.tensor([ms, ms_e2e], device=dev)
@@ -613,7 +641,11 @@ def main():
     ap.add_argument("--no-direct-grads", action="store_true", help="let autograd accumulate parameter gradients (A/B switch)")
     ap.add_argument("--no-overlap", action="store_true", help="N > 1: one all-reduce after backward instead of overlapped chunks")
     ap.add_argument("--no-secondary", action="store_true", help="skip the ReXNet-1.0x leg (BASELINE configs[1]) at N=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss and the model state it left as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.config:
         args.model = {1: "rexnet1_0x", 2: "repvgg_a1", 3: "yolov4", 4: "unet3p"}[args.config]
 
@@ -627,6 +659,8 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("bench.py (impl b200) needs a CUDA device: there is no CPU fallback")
     if args.micro:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: --micro runs no training step")
         from tools.micro_bench import run_micro
         if rank == 0:
             print(json.dumps(run_micro(measured_peaks())), flush=True)
@@ -648,7 +682,7 @@ def main():
             gc.collect()
             torch.cuda.empty_cache()
             sargs = argparse.Namespace(**vars(args))
-            sargs.steps, sargs.warmup, sargs.batch = 10, 3, 0
+            sargs.steps, sargs.warmup, sargs.batch, sargs.dump_outputs = 10, 3, 0, None
             sec = measure(sargs, Workload("rexnet1_0x"), 0, local_rank, 1, full=False)
             result["secondary"] = {"workload": sec["config"]["workload"] + ", batch 256, CUDA-graph replay, inputs resident in HBM",
                                    "images_per_s": sec["value"], "ms_per_step": sec["ms_per_step"], "steps": sec["steps"],

@@ -92,18 +92,18 @@ class FlakyCrossEntropy(nn.CrossEntropyLoss):
         return loss * float("nan") if self.calls == self.bad else loss
 
 
-def run_scenarios(T, record):
+def run_scenarios(T, record, output_file):
     """Drives the trainer classes of namespace ``T`` (reference or this package) through every scenario; ``record(tag, dict)``
-    stores the observable results."""
+    stores the observable results. The trainers write their checkpoints to ``output_file``."""
     sd = lambda m: {k: v.detach().clone() for k, v in m.state_dict().items()}   # noqa: E731
     # 1. classification: two epochs, one-cycle schedule, gradient accumulation + clipping
     model = cls_model()
     seen = []
     tr = T.ClassificationTrainer(model, cls_batches(6, 1), cls_batches(3, 2), nn.CrossEntropyLoss(),
-                                 torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file="/tmp/_hb_trainers_ckpt.pth",
+                                 torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file=output_file,
                                  gradient_acc=2, gradient_clip=0.5, on_epoch_end=lambda m: seen.append(dict(m)))
     tr.fit_n_epochs(2, 3e-3, sched_type="onecycle")
-    ckpt = torch.load("/tmp/_hb_trainers_ckpt.pth", map_location="cpu")
+    ckpt = torch.load(output_file, map_location="cpu")
     record("cls_fit", dict(metrics=seen, state=sd(model), step=tr.step, epoch=tr.epoch, min_loss=tr.min_loss,
                            ckpt_keys=sorted(ckpt), ckpt_epoch=ckpt["epoch"], ckpt_step=ckpt["step"],
                            msg=tr._eval_metrics_str(seen[-1])))
@@ -112,7 +112,7 @@ def run_scenarios(T, record):
     data = cls_batches(5, 3)
     tr = T.ClassificationTrainer(model, data, cls_batches(2, 4), FlakyCrossEntropy(bad=3),
                                  torch.optim.SGD(model.parameters(), lr=1e-2, momentum=0.9, weight_decay=1e-2), gpu=None,
-                                 output_file="/tmp/_hb_trainers_ckpt.pth", skip_nan_loss=True)
+                                 output_file=output_file, skip_nan_loss=True)
     tr.fit_n_epochs(1, 5e-2, freeze_until="0", sched_type="cosine", norm_weight_decay=0.0)
     record("cls_frozen_cosine", dict(state=sd(model), groups=[(len(g["params"]), g["weight_decay"]) for g in tr.optimizer.param_groups],
                                      frozen=[n for n, p in model.named_parameters() if not p.requires_grad], step=tr.step,
@@ -120,14 +120,14 @@ def run_scenarios(T, record):
     # 3. binary classification
     model = cls_model(1)
     tr = T.BinaryClassificationTrainer(model, cls_batches(4, 5, binary=True), cls_batches(2, 6, binary=True), nn.BCEWithLogitsLoss(),
-                                       torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file="/tmp/_hb_trainers_ckpt.pth")
+                                       torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file=output_file)
     tr.fit_n_epochs(1, 1e-2)
     m = tr.evaluate()
     record("binary", dict(state=sd(model), metrics=m, msg=tr._eval_metrics_str(m)))
     # 4. segmentation
     model = seg_model()
     tr = T.SegmentationTrainer(model, seg_batches(3, 7), seg_batches(2, 8), nn.CrossEntropyLoss(ignore_index=255),
-                               torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file="/tmp/_hb_trainers_ckpt.pth",
+                               torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file=output_file,
                                num_classes=5)
     tr.fit_n_epochs(1, 1e-2)
     m = tr.evaluate()
@@ -136,7 +136,7 @@ def run_scenarios(T, record):
     loader, detections = det_data()
     model = FixedDetector(detections)
     tr = T.DetectionTrainer(model, loader, loader, None, torch.optim.SGD(model.parameters(), lr=1e-2), gpu=None,
-                            output_file="/tmp/_hb_trainers_ckpt.pth")
+                            output_file=output_file)
     tr.fit_n_epochs(1, 1e-2)
     m = tr.evaluate()
     assign_iou = getattr(T, "assign_iou", None) or __import__(T.__name__ + ".detection", fromlist=["assign_iou"]).assign_iou
@@ -146,7 +146,7 @@ def run_scenarios(T, record):
     # 6. learning-rate finder and set-up check
     model = cls_model()
     tr = T.ClassificationTrainer(model, cls_batches(8, 9), cls_batches(2, 10), nn.CrossEntropyLoss(),
-                                 torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file="/tmp/_hb_trainers_ckpt.pth")
+                                 torch.optim.Adam(model.parameters(), lr=1e-3), gpu=None, output_file=output_file)
     tr.find_lr(start_lr=1e-5, end_lr=1e-1, num_it=6)
     rec = dict(lrs=list(tr.lr_recorder), losses=list(tr.loss_recorder))
     tr.check_setup(lr=1e-3, num_it=4)

@@ -331,7 +331,7 @@ if __name__ == "__main__" and "--optim2" in sys.argv:
     print("optim2.pt", (OUT / "optim2.pt").stat().st_size)
 
 
-if __name__ == "__main__" and not any(f in sys.argv for f in ("--zoo", "--zoo-resnet", "--zoo-f3", "--zoo-f3b", "--yolo", "--trainers", "--seg", "--api", "--trainer", "--optim2")):
+if __name__ == "__main__" and not any(f in sys.argv for f in ("--zoo", "--zoo-resnet", "--zoo-f3", "--zoo-f3b", "--yolo", "--trainers", "--seg", "--api", "--trainer", "--optim2", "--cross")):
     gen_activations()
     gen_losses()
     gen_boxes()
@@ -769,8 +769,10 @@ def gen_trainers():
     T = importlib.import_module("holocron.trainer")
     sys.path.insert(0, str(ROOT / "tests"))
     import _trainer_cases as cases
+    import tempfile
     d = {}
-    cases.run_scenarios(T, lambda tag, rec: d.__setitem__(tag, rec))
+    with tempfile.TemporaryDirectory() as tmp:
+        cases.run_scenarios(T, lambda tag, rec: d.__setitem__(tag, rec), str(Path(tmp) / "ckpt.pth"))
     torch.save(d, OUT / "trainers.pt")
 
 
@@ -809,3 +811,77 @@ def gen_seg():
 if __name__ == "__main__" and "--seg" in sys.argv:
     gen_seg()
     print("zoo_seg.pt", (OUT / "zoo_seg.pt").stat().st_size)
+
+
+# ------------------------------------------------------------------------------------------------ module / format cross-checks
+def gen_cross():
+    """What the reference's own PyConv2d / TridentConv2d / ConcatDownsample2d modules, its Mixup collate and its hub loader
+    produce on seeded inputs -> tests/golden/cross_checks.pt (tests/test_zoo_wiring_cpu.py, tests/test_host_logic.py,
+    tests/test_formats_cpu.py compare against it)."""
+    import importlib.util
+    import types
+    for name in ("matplotlib", "matplotlib.pyplot", "tqdm", "tqdm.auto"):     # plots / progress bars of holocron.utils only
+        try:
+            missing = name not in sys.modules and importlib.util.find_spec(name) is None
+        except (ImportError, ValueError):
+            missing = True
+        if missing:
+            stub = types.ModuleType(name)
+            stub.tqdm = lambda it, *a, **k: it
+            sys.modules[name] = stub
+    d = {}
+    g = torch.Generator().manual_seed(20)
+    x = torch.rand(2, 8, 8, 8, generator=g)
+    pyconv = []
+    for kwargs in (dict(num_levels=1), dict(num_levels=2), dict(num_levels=3, groups=[1, 2, 4]), dict(num_levels=4, stride=2)):
+        torch.manual_seed(0)
+        ref = holocron.nn.PyConv2d(8, 16, 3, padding=1, **kwargs)
+        pyconv.append(dict(kwargs=kwargs, params=[p.detach().clone() for p in ref.parameters()], num_levels=ref.num_levels,
+                           out=ref(x).detach()))
+    d["pyconv"] = dict(x=x, cases=pyconv)
+    from holocron.models.classification.tridentnet import TridentConv2d as RefTrident
+    x3 = torch.rand(1, 24, 8, 8, generator=g)
+    trident = []
+    for k, dil in ((1, 1), (3, 3)):
+        torch.manual_seed(1)
+        ref = RefTrident(8, 8, k, padding=k // 2, dilation=dil, bias=False)
+        trident.append(dict(k=k, dil=dil, state={n: v.clone() for n, v in ref.state_dict().items()}, out=ref(x3).detach()))
+    d["trident"] = dict(x=x3, cases=trident)
+    xc = torch.rand(2, 6, 8, 12, generator=g)
+    d["concat_downsample"] = dict(x=xc, out=holocron.nn.ConcatDownsample2d(2)(xc))
+    from holocron.utils.data import Mixup as RefMixup
+    mixup = []
+    for num_classes, alpha, seed in ((7, 0.2, 0), (7, 1.0, 1), (1, 0.4, 2)):
+        gm = torch.Generator().manual_seed(seed)
+        xm = torch.rand(6, 3, 5, 5, generator=gm)
+        tm = torch.randint(0, max(num_classes, 2), (6,), generator=gm)
+        torch.manual_seed(100 + seed)
+        xr, tr = RefMixup(num_classes, alpha)(xm.clone(), tm.clone())
+        mixup.append(dict(num_classes=num_classes, alpha=alpha, seed=seed, x=xm, t=tm, x_out=xr, t_out=tr))
+    d["mixup"] = mixup
+    # hub format: the architecture keys the reference's model_from_hf_hub resolves (holocron.models.__dict__[cfg["arch"]]) and
+    # the state_dict layout its strict load_state_dict accepts for a 10-class rexnet1_0x, read back through that loader
+    import json
+    import tempfile
+    ref_utils = holocron.models.utils
+    torch.manual_seed(4)
+    src = holocron.models.rexnet1_0x(num_classes=10)
+    with tempfile.TemporaryDirectory() as tmp:
+        folder = Path(tmp)
+        (folder / "config.json").write_text(json.dumps({"arch": "rexnet1_0x", "classes": [str(i) for i in range(10)]}))
+        torch.save(src.state_dict(), folder / "pytorch_model.bin")
+        orig = ref_utils.hf_hub_download
+        ref_utils.hf_hub_download = lambda repo_id, filename, **kw: str(folder / filename)
+        try:
+            loaded = ref_utils.model_from_hf_hub("frgfm/rexnet1_0x")
+        finally:
+            ref_utils.hf_hub_download = orig
+    d["hub"] = dict(arch="rexnet1_0x", num_classes=10,
+                    registry=sorted(k for k, v in vars(holocron.models).items() if callable(v) and not k.startswith("_")),
+                    layout=[(k, tuple(v.shape), v.dtype) for k, v in loaded.state_dict().items()])
+    torch.save(d, OUT / "cross_checks.pt")
+
+
+if __name__ == "__main__" and "--cross" in sys.argv:
+    gen_cross()
+    print("cross_checks.pt", (OUT / "cross_checks.pt").stat().st_size)

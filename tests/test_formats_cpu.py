@@ -2,7 +2,7 @@
 
   * the HF-hub repository layout of reference models/utils.py:146-175 (config.json + pytorch_model.bin), written by
     ``save_hf_hub_folder`` and read back by ``model_from_hf_hub`` through a stubbed ``hf_hub_download`` (no network);
-    the same two files are read by the UNMODIFIED reference's ``model_from_hf_hub`` when /root/reference is mounted;
+    the same two files match what the UNMODIFIED reference's ``model_from_hf_hub`` reads (tests/golden/cross_checks.pt);
   * ``load_pretrained_params`` (reference models/utils.py:89-113) from a ``file://`` URL incl. key filter / replacement, and
     the factories' ``checkpoint=Checkpoint(...)`` argument;
   * ``clean_checkpoint`` (reference references/clean_checkpoint.py): Trainer checkpoint -> bare legacy-serialised state_dict."""
@@ -16,7 +16,7 @@ import torch
 import holocron_b200 as hb
 from holocron_b200.models import checkpoints as CK
 from holocron_b200.models import utils as U
-from oracle import reference_loader
+from conftest import load_golden
 
 
 def _stub_hub(monkeypatch, folder, repo):
@@ -43,25 +43,29 @@ def test_hf_hub_folder_round_trip(tmp_path, monkeypatch):
     assert list(sd) == list(sl) and all(torch.equal(sd[k], sl[k]) for k in sd)
 
 
-@pytest.mark.skipif(not reference_loader.available(), reason="needs /root/reference (build container only)")
 def test_hf_hub_folder_is_readable_by_the_reference(tmp_path, monkeypatch):
-    """Interoperability both ways: a folder written here loads in the unmodified reference (same arch registry key, same
-    parameter names), and a folder holding the reference's state_dict loads here."""
-    holocron = reference_loader.load()
+    """Interoperability both ways, against the reference's hub loader as recorded in tests/golden/cross_checks.pt
+    (make_golden.py --cross): a folder written here names an architecture the reference registers and holds exactly the
+    parameter names, shapes and dtypes its strict ``load_state_dict`` accepts, and a folder holding a state_dict in the
+    reference's layout loads here."""
+    ref = load_golden("cross_checks")["hub"]
     torch.manual_seed(4)
-    ours = hb.models.rexnet1_0x(num_classes=10)
-    classes = [str(i) for i in range(10)]
+    ours = hb.models.rexnet1_0x(num_classes=ref["num_classes"])
+    classes = [str(i) for i in range(ref["num_classes"])]
     folder = U.save_hf_hub_folder(ours, tmp_path / "hub", "rexnet1_0x", classes)
-    ref_utils = holocron.models.utils
-    monkeypatch.setattr(ref_utils, "hf_hub_download", lambda repo_id, filename, **kw: str(folder / filename))
-    ref_model = ref_utils.model_from_hf_hub("frgfm/rexnet1_0x")
-    so, sr = ours.state_dict(), ref_model.state_dict()
-    assert list(so) == list(sr) and all(torch.equal(so[k], sr[k]) for k in so)
-    # and back: the reference's state_dict in the same layout
-    torch.save(ref_model.state_dict(), folder / "pytorch_model.bin")
+    # what the reference's model_from_hf_hub reads: cfg["arch"] from its registry, len(cfg["classes"]), the state_dict
+    cfg = json.loads((folder / "config.json").read_text())
+    assert cfg["arch"] == ref["arch"] and cfg["arch"] in ref["registry"] and len(cfg["classes"]) == ref["num_classes"]
+    sd = torch.load(folder / "pytorch_model.bin", map_location="cpu")
+    assert [(k, tuple(v.shape), v.dtype) for k, v in sd.items()] == ref["layout"]
+    # and back: a state_dict in the reference's layout, seeded values
+    g = torch.Generator().manual_seed(5)
+    theirs = {k: (torch.rand(shape, generator=g) * 2 - 1).to(dtype) if dtype.is_floating_point else
+              torch.randint(0, 100, shape, generator=g).to(dtype) for k, shape, dtype in ref["layout"]}
+    torch.save(theirs, folder / "pytorch_model.bin")
     _stub_hub(monkeypatch, folder, "frgfm/rexnet1_0x")
     back = U.model_from_hf_hub("frgfm/rexnet1_0x")
-    assert all(torch.equal(v, back.state_dict()[k]) for k, v in sr.items())
+    assert all(torch.equal(v, back.state_dict()[k]) for k, v in theirs.items())
 
 
 def _checkpoint(url, arch):

@@ -418,16 +418,8 @@ def test_f3b_classification_batch_statistics(name):
 SEG = load_golden("zoo_seg")
 
 
-# unet_rexnet13 (ReXNet-1.3x taps: 35 / 61 / ... channels, convolution + bias + SiLU units without normalisation) failed in the
-# session's last GPU run inside the stand-alone activation pass (channels % 8 != 0); conv2d_bias_act now activates the zero-padded
-# output and slices afterwards, but there was no GPU time left to re-run it: its tree is pinned on the CPU
-# (tests/test_zoo_wiring_cpu.py), the GPU case is skipped rather than claimed.
-_SEG_GPU = [pytest.param(n, marks=pytest.mark.skip(reason="fix not re-run on a GPU (budget)")) if n == "unet_rexnet13" else n
-            for n in C.SEG]
-
-
 @pytest.mark.parametrize("mode", ["eval", "train"])
-@pytest.mark.parametrize("name", _SEG_GPU)
+@pytest.mark.parametrize("name", list(C.SEG))
 def test_unet_family(name, mode):
     """U-Net / UNet+ / UNet++ / DynamicUNet (own encoder, ReXNet-1.3x encoder) against the reference's fp32 fixtures: frozen
     normalisation: logits <= 2e-2, loss <= 1e-2, last-layer gradient <= 5e-2, first / middle by the autocast-twin rule; batch

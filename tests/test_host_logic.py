@@ -163,13 +163,14 @@ def test_remaining_optimizer_constructors_validate_like_the_reference():
         hb.optim.Adan(w).step()
 
 
-def test_mixup_collate_matches_reference_draw_for_draw(monkeypatch):
+def test_mixup_collate_matches_reference_draw_for_draw():
     """holocron.utils.data.Mixup (reference utils/data/collate.py:16-64): same one-hot encoding, same RNG draws in the same
-    order (Beta sample, permutation), same in-place mixing - seeded batches come out identical to the unmodified reference's."""
+    order (Beta sample, permutation), same in-place mixing - seeded batches come out identical to what the unmodified
+    reference's Mixup returned on them (tests/golden/make_golden.py --cross)."""
     import pytest
     import torch
     import holocron_b200 as hb
-    from oracle import reference_loader
+    from conftest import load_golden
     with pytest.raises(ValueError):
         hb.utils.data.Mixup(10, alpha=-0.1)
     mix = hb.utils.data.Mixup(num_classes=7, alpha=0.0)
@@ -177,28 +178,7 @@ def test_mixup_collate_matches_reference_draw_for_draw(monkeypatch):
     xo, to = mix(x.clone(), t)
     assert torch.equal(xo, x) and to.shape == (4, 7) and to.dtype == x.dtype and torch.equal(to.argmax(1), t)
     assert hb.utils.data.Mixup(1, 0.0)(x.clone(), torch.tensor([1, 0, 1, 1]))[1].shape == (4, 1)
-    if not reference_loader.available():
-        pytest.skip("needs /root/reference (build container only)")
-    import sys
-    import types
-    for name in ("matplotlib", "matplotlib.pyplot", "tqdm", "tqdm.auto"):     # plots / progress bars of holocron.utils.misc only
-        import importlib.util
-        try:
-            missing = name not in sys.modules and importlib.util.find_spec(name) is None
-        except (ImportError, ValueError):
-            missing = True
-        if missing:                                          # only what this image really lacks (matplotlib), never a real package
-            stub = types.ModuleType(name)
-            stub.tqdm = lambda it, *a, **k: it
-            monkeypatch.setitem(sys.modules, name, stub)     # undone after the test: later tests must not see the stubs
-    reference_loader.load()
-    from holocron.utils.data import Mixup as RefMixup
-    for num_classes, alpha, seed in ((7, 0.2, 0), (7, 1.0, 1), (1, 0.4, 2)):
-        g = torch.Generator().manual_seed(seed)
-        x = torch.rand(6, 3, 5, 5, generator=g)
-        t = torch.randint(0, max(num_classes, 2), (6,), generator=g)
-        torch.manual_seed(100 + seed)
-        xr, tr = RefMixup(num_classes, alpha)(x.clone(), t.clone())
-        torch.manual_seed(100 + seed)
-        xm, tm = hb.utils.data.Mixup(num_classes, alpha)(x.clone(), t.clone())
-        assert torch.equal(xr, xm) and torch.equal(tr, tm)
+    for case in load_golden("cross_checks")["mixup"]:
+        torch.manual_seed(100 + case["seed"])
+        xm, tm = hb.utils.data.Mixup(case["num_classes"], case["alpha"])(case["x"].clone(), case["t"].clone())
+        assert torch.equal(case["x_out"], xm) and torch.equal(case["t_out"], tm)

@@ -31,9 +31,9 @@ def _same_state(got, want, tol=1e-5):
 
 
 @pytest.fixture(scope="module")
-def runs():
+def runs(tmp_path_factory):
     ours = {}
-    cases.run_scenarios(hb.trainer, lambda tag, rec: ours.__setitem__(tag, rec))
+    cases.run_scenarios(hb.trainer, lambda tag, rec: ours.__setitem__(tag, rec), str(tmp_path_factory.mktemp("trainers") / "ckpt.pth"))
     return ours, load_golden("trainers")
 
 
